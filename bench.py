@@ -5,6 +5,7 @@
     python bench.py --impl reference --steps K --warmup W     # CPU restatement of the reference path
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
            --master-port P bench.py --gpus N --steps K --warmup W
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR   # also write the last timed step's outputs
 
 Metric (BASELINE.json): examples/sec (fwd+bwd) DeepFM batch=65536.  Workload at N=1 = config C2:
 26 categorical slots x 1M-row tables, D=16, batch 65536, DNN [256,32]->1, synthetic uniform ids,
@@ -31,6 +32,9 @@ C2 = dict(slots=26, rows=1_000_000, dim=16, batch=65536, dnn=[256, 32])
 # the ranks (strong scaling in the batch), rows sharded row-wise with the fused NVLink peer-memory gather / update.
 # The tower is not specified by BASELINE.json; [512, 256] -> 1 is this repo's choice.
 C5 = dict(slots=26, rows=3_846_154, dim=128, batch=65536, dnn=[512, 256])
+# --dump-outputs writes the embedding vectors of a fixed, seeded sample of table rows, this many bytes of them: the tables
+# themselves are 1.7 GB at C2 and 51 GB at C5
+DUMP_EMBED_BYTES = 16 << 20
 
 
 def measured_peaks():
@@ -122,6 +126,35 @@ def run_reference(args):
     print(json.dumps(line), flush=True)
 
 
+def dump_outputs(trainer, out_dir):
+    """Writes what the trainer's last step left for its caller as float32 DIR/<name>.npy: the step's loss and
+    probabilities, the dense tower, the FM bias, and the embedding vectors and first-order weights of a fixed sample of
+    table rows (row indices drawn with seed 0, sorted), so that two builds run with the same arguments can be compared
+    array for array.  main() calls it right after the timed loop and before the end-to-end passes step the trainer again:
+    that order is what makes the files hold the last timed step.
+
+    Under --optimizer adam_rows_tf the tables lag the rows' pending Adam steps, so this first replays them in place
+    (flush_optimizer, what a caller does before reading the tables; a no-op for the other optimizers).  The end-to-end
+    and per-kernel passes that follow then start with no pending steps, unlike a run without --dump-outputs; the
+    headline timed region is not affected."""
+    import numpy as np
+    import torch
+    trainer.flush_optimizer()
+    coll = trainer.coll
+    n = min(coll.total_rows, DUMP_EMBED_BYTES // (4 * coll.dim))
+    rows = np.sort(np.random.default_rng(0).choice(coll.total_rows, n, replace=False))
+    rows = torch.from_numpy(rows).to(coll.weight.device)
+    out = {"loss": trainer.loss, "prob": trainer.prob, "fm_bias": coll.bias,
+           "embed_rows": coll.emb_view().index_select(0, rows), "linear_rows": coll.lin_view().index_select(0, rows)}
+    for i, (w, b) in enumerate(zip(trainer.w, trainer.b)):
+        out[f"dense{i}_kernel"] = w
+        if b is not None:
+            out[f"dense{i}_bias"] = b
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in out.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.detach().float().cpu().numpy())
+
+
 def workload_config(n, name="c2"):
     if name == "c5":
         return {"workload": f"C5 DLRM-shape DeepFM: {C5['slots']} slots x {C5['rows']} rows (100M total), D={C5['dim']}, "
@@ -159,11 +192,18 @@ def main():
     ap.add_argument("--dw-first", type=int, default=0, help="N=1: enqueue the layer-0 dW GEMM before the embedding update")
     ap.add_argument("--exchange", default="p2p", choices=["p2p", "nccl"],
                     help="N>1: fused NVLink peer-memory gather/update (p2p) or NCCL all-to-all pipeline (nccl)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="N=1: after the timed steps, write what the last one computed to DIR/<name>.npy (float32): loss, "
+                         "probabilities, dense tower, FM bias and a fixed seeded sample of the embedding rows")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.dump_outputs and (args.impl != "ours" or world > 1):
+        ap.error("--dump-outputs needs --impl ours in a single process")
 
     if args.impl == "reference":
         if rank == 0:
@@ -271,6 +311,8 @@ def main():
         barrier()
     ms = max_over_ranks(e0.elapsed_time(e1))
     value = B * world * args.steps / (ms * 1e-3)
+    if args.dump_outputs:               # before the end-to-end passes below step the trainer again
+        dump_outputs(trainer, args.dump_outputs)
     final_loss = float(trainer.loss.item())
 
     # ---- end-to-end: host buffers in, loss out, copies inside the timed region --------------------

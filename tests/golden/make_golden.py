@@ -1,9 +1,9 @@
 """Generates tests/golden/hotpath_golden_{f32,f64}.npz by EXECUTING THE REFERENCE'S OWN SOURCE FILES
-(read from /root/reference, never copied) under the numpy-backed `tensorflow` stand-in in
-oracle/tf_shim.  Run here (the CPU container); the .npz files are committed and travel to the GPU
-box, /root/reference does not.
+(read from a checkout of the original deep_recommenders project, never copied) under the numpy-backed
+`tensorflow` stand-in in oracle/tf_shim.  Needs no GPU.  The .npz files are committed and the tests
+read only them; rerun this by hand when the golden cases change.
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py <checkout of the original deep_recommenders project>
 
 What executes from the reference:
   keras/models/ranking/fm.py        FM.call (:23-37), FactorizationMachine.call (:54-63)
@@ -26,7 +26,9 @@ import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
-REFERENCE = os.environ.get("DR_REFERENCE", "/root/reference")
+if len(sys.argv) != 2 or not os.path.isdir(os.path.join(sys.argv[1], "deep_recommenders")):
+    sys.exit("usage: python tests/golden/make_golden.py <checkout of the original deep_recommenders project>")
+REFERENCE = os.path.abspath(sys.argv[1])
 sys.path.insert(0, os.path.join(ROOT, "oracle", "tf_shim"))
 sys.path.insert(0, REFERENCE)
 sys.dont_write_bytecode = True

@@ -99,6 +99,34 @@ def test_bench_reference_arm_json_contract():
     assert line["e2e"]["h2d_bytes_per_step"] == 0 and line["higher_is_better"] is True
 
 
+def test_bench_dump_outputs_writes_float32_arrays_of_a_fixed_row_sample(tmp_path, monkeypatch):
+    """`bench.py --dump-outputs DIR` (on a stand-in trainer over CPU tensors): every array is a float32 .npy, two dumps of
+    the same state are identical, and the embedding sample holds distinct table rows in ascending order with their own
+    first-order weights."""
+    import os
+    import types
+    import bench
+    from deep_recommenders_b200.embedding import EmbeddingCollection
+    coll = EmbeddingCollection([1000, 2000, 500], 16, device="cpu", seed=1)
+    with torch.no_grad():
+        coll.lin_view().copy_(torch.arange(coll.total_rows, dtype=torch.float32))
+    trainer = types.SimpleNamespace(coll=coll, loss=torch.ones(1), prob=torch.rand(64), w=[torch.rand(48, 8), torch.rand(8, 1)],
+                                    b=[torch.rand(8), None], flush_optimizer=lambda: None)
+    monkeypatch.setattr(bench, "DUMP_EMBED_BYTES", 64 * 16 * 4)
+    bench.dump_outputs(trainer, str(tmp_path / "a"))
+    bench.dump_outputs(trainer, str(tmp_path / "b"))
+    names = sorted(os.listdir(tmp_path / "a"))
+    assert names == ["dense0_bias.npy", "dense0_kernel.npy", "dense1_kernel.npy", "embed_rows.npy", "fm_bias.npy",
+                     "linear_rows.npy", "loss.npy", "prob.npy"]
+    for n in names:
+        a = np.load(tmp_path / "a" / n)
+        assert a.dtype == np.float32 and np.array_equal(a, np.load(tmp_path / "b" / n)), n
+    idx = np.load(tmp_path / "a" / "linear_rows.npy").astype(np.int64)
+    assert len(idx) == 64 and np.all(np.diff(idx) > 0)
+    assert np.array_equal(np.load(tmp_path / "a" / "embed_rows.npy"), coll.emb_view().detach().numpy()[idx])
+    np.testing.assert_array_equal(np.load(tmp_path / "a" / "dense0_kernel.npy"), trainer.w[0].numpy())
+
+
 def test_ctypes_signatures_match_the_header_arity_and_pointer_kinds():
     """Every entry of _lib._SIGS must have exactly the parameters its declaration in include/deeprec_b200.h has, with
     pointers bound as pointers, 64-bit integers as c_int64, ints as c_int and floats as c_float (an ABI drift here

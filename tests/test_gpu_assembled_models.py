@@ -53,11 +53,12 @@ def test_dcn_step_matches_oracle(B, S, D, units, ncross, alpha):
     y = rng.integers(0, 2, (B, 1)).astype(np.float32)
     idt, yt = torch.from_numpy(ids).cuda(), torch.from_numpy(y).cuda()
     z = model.logits(idt)                                     # builds the lazily created layers
+    gen = torch.Generator(device="cuda").manual_seed(B + S)   # not the global generator: its state depends on earlier tests
     with torch.no_grad():                                     # zero-init biases would hide bias-path errors
         for c in model.cross:
-            c.bias.normal_(0, 0.1)
+            c.bias.normal_(0, 0.1, generator=gen)
         for l in model.dnn.layers:
-            l.bias.normal_(0, 0.1)
+            l.bias.normal_(0, 0.1, generator=gen)
     model.zero_grad()
     z = model.logits(idt)
     loss = torch.nn.functional.binary_cross_entropy_with_logits(z, yt, reduction="sum")
@@ -76,9 +77,23 @@ def test_dcn_step_matches_oracle(B, S, D, units, ncross, alpha):
         xs.append(nxt)
     dw = [npy(l.kernel).astype(F64) for l in model.dnn.layers]
     db = [npy(l.bias).astype(F64) for l in model.dnn.layers]
+    # ReLU masks: a unit whose pre-activation lies within rounding of 0 (the float32 forward against this float64 one)
+    # may fall on either side, and one such unit moves a whole batch row's term in the weight-gradient column it feeds.
+    # Those units take the side the GPU forward took; every other unit's side must agree with the float64 forward.
+    with torch.no_grad():
+        h_gpu = model.embeddings(idt, want_logit=False)[0].view(B, -1)
     hs = [x0]
-    for w, b in zip(dw, db):
-        hs.append(R.dense(hs[-1], w, b, "relu", F64))
+    for w, b, layer in zip(dw, db, model.dnn.layers):
+        zpre = R.dense(hs[-1], w, b, None, F64)
+        with torch.no_grad():
+            h_gpu = layer(h_gpu)
+        on = npy(h_gpu) > 0
+        near0 = np.abs(zpre) <= 2e-5 * (np.abs(hs[-1]) @ np.abs(w) + np.abs(b))
+        assert np.array_equal(on[~near0], zpre[~near0] > 0), "ReLU pattern differs from the float64 forward"
+        h = np.maximum(zpre, 0)
+        h[near0 & on] = np.maximum(zpre[near0 & on], np.finfo(F64).tiny)
+        h[near0 & ~on] = 0.0
+        hs.append(h)
     hw, hb = npy(model.head.kernel).astype(F64), npy(model.head.bias).astype(F64)
     feat = np.concatenate([xs[-1], hs[-1]], axis=1)
     z_ref = feat @ hw + hb
